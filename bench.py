@@ -3,7 +3,7 @@
 with the float CPU implementation timed beside it.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--model tiny|base|..] [--batch B]
-                    [--headline-only]
+                    [--headline-only] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of B synthetic 10 s @ 16 kHz utterances.
 
@@ -20,6 +20,10 @@ collective; the headline stays tiny / 32 per GPU so the driver's scaling efficie
 --impl reference: the CPU arm -- the Hugging Face float implementation of the same model (the graphs the reference
 ships were exported from it), same seeded weights and inputs, ALL host cores, the headline's batch of 32 as one
 batch per step (plus the reference's own batch-1 serial operating point, reported inside `cpu_baseline`).
+
+--dump-outputs DIR: after the timed steps, write the token ids the device-resident path returned in its last timed
+step as DIR/<config>_tokens.npy (rank 0's utterances), so that two builds can be compared output for output: the
+weights and the audio are seeded, so the inputs are the same in every run with the same arguments.
 """
 import argparse
 import json
@@ -240,7 +244,7 @@ def measure_config(api, torch, dist, model, B, steps, warmup, rank, world, local
         torch.cuda.synchronize()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record(stream)
-        tr.transcribe_device(dev.data_ptr(), N_SAMPLES, lengths)
+        toks = tr.transcribe_device(dev.data_ptr(), N_SAMPLES, lengths)
         e1.record(stream)
         e1.synchronize()
         ev_ms.append(e0.elapsed_time(e1))
@@ -307,6 +311,16 @@ def measure_config(api, torch, dist, model, B, steps, warmup, rank, world, local
     return rec, toks, audios
 
 
+def dump_outputs(out_dir, outputs):
+    """Token ids per operating point as float64 [utterances, longest], padded with -1 (ids are exact in float64)."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, toks in outputs.items():
+        a = np.full((len(toks), max(len(t) for t in toks)), -1.0)
+        for i, t in enumerate(toks):
+            a[i, :len(t)] = t
+        np.save(os.path.join(out_dir, f"{name}_tokens.npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -317,7 +331,11 @@ def main():
     ap.add_argument("--batch", type=int, default=32)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--headline-only", action="store_true", help="skip the other BASELINE configs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the token ids of each config's last timed step to DIR/<config>_tokens.npy")
     args = ap.parse_args()
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs applies to the GPU path")
     if args.impl == "reference":
         run_reference(args)
         return
@@ -342,6 +360,7 @@ def main():
     wall0 = time.perf_counter()
     head, toks, audios = measure_config(api, torch, dist, model, B, args.steps, args.warmup, rank, world, local)
     wall_head = time.perf_counter() - wall0
+    outputs = {f"{model}_b{B}": toks}
 
     # ---- the other BASELINE operating points (same run, same box) ----
     configs = {}
@@ -349,12 +368,12 @@ def main():
     if default_headline and not args.headline_only:
         extra = []
         if world == 1:
-            extra = [("tiny_b1", "tiny", 1, 10, 3), ("base_b256", "base", 256, 3, 2), ("base_streaming_b64", "base_streaming", 64, 3, 2)]
+            extra = [("tiny_b1", "tiny", 1), ("base_b256", "base", 256), ("base_streaming_b64", "base_streaming", 64)]
         elif world == 8:
-            extra = [("base_b2048_8gpu", "base", 256, 3, 2)]
-        for key, m2, b2, k2, w2 in extra:
+            extra = [("base_b2048_8gpu", "base", 256)]
+        for key, m2, b2 in extra:
             try:
-                rec, _, _ = measure_config(api, torch, dist, m2, b2, k2, w2, rank, world, local)
+                rec, outputs[key], _ = measure_config(api, torch, dist, m2, b2, args.steps, args.warmup, rank, world, local)
                 configs[key] = rec
             except Exception as e:  # an extra config must never take the headline down
                 configs[key] = {"error": f"{type(e).__name__}: {e}"}
@@ -404,6 +423,8 @@ def main():
                 line["cpu_baseline"] = {"value": np_ups, "unit": "utt/s", "cores": min(threads, 16), "kind": "port",
                                         "sample": f"1 utterance, numpy oracle (HF arm failed: {type(e).__name__}: {e})",
                                         "tokens_match_gpu": bool(np_toks == toks[0])}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

@@ -1,100 +1,36 @@
 """GPU: key-term biasing on a streaming architecture through the reference ABI (`keyterms` / `keyterm_boost`
 options and moonshine_transcriber_set_keyterms).  Expected text: the streaming oracle's logits with the
-REFERENCE's own ContextBiaser (oracle/_ref, compiled from core/context-biaser.cpp) applied before each argmax,
-key terms spelled by the reference's own tokenizer."""
-import ctypes
-import os
-
-import numpy as np
+REFERENCE's own ContextBiaser (core/context-biaser.cpp) applied before each argmax, key terms spelled by the
+reference's own tokenizer; the resulting ids are stored in golden/ref_keyterms.json by
+golden/make_golden_reference.py."""
 import pytest
 
 from moonshine_b200 import api
 from moonshine_b200.arch import ARCHS
-from moonshine_b200.weights import synth_audio, synth_tokenizer_bin, synth_weights
-from oracle import build_ref
+from moonshine_b200.weights import synth_audio, synth_tokenizer_bin
 from oracle import moonshine_oracle as orc
-from oracle.moonshine_streaming_oracle import SDims, StreamingOracle
-from tests.util import memory_files
+from tests.util import memory_files, reference_golden
 
 pytestmark = pytest.mark.gpu
+
+KEYTERM_AUDIO = (21, 16000 * 3)
 
 
 @pytest.fixture(scope="module")
 def ref():
-    path = build_ref.build()
-    if path is None or not os.path.exists(path):
-        pytest.skip("oracle/_ref not available")
-    lib = ctypes.CDLL(path)
-    c = ctypes
-    lib.ref_tokenizer_new_bpe.restype = c.c_void_p
-    lib.ref_tokenizer_new_bpe.argtypes = [c.c_char_p, c.c_uint64]
-    lib.ref_text_to_tokens.restype = c.c_int32
-    lib.ref_text_to_tokens.argtypes = [c.c_void_p, c.c_char_p, c.POINTER(c.c_int32), c.c_int32]
-    lib.ref_biaser_new.restype = c.c_void_p
-    lib.ref_biaser_add.argtypes = [c.c_void_p, c.POINTER(c.c_int32), c.c_int32]
-    lib.ref_biaser_reset.argtypes = [c.c_void_p]
-    lib.ref_biaser_advance.argtypes = [c.c_void_p, c.c_int32]
-    lib.ref_biaser_apply.argtypes = [c.c_void_p, c.POINTER(c.c_float), c.c_int32]
-    lib.ref_biaser_variants.restype = c.c_int32
-    lib.ref_biaser_variants.argtypes = [c.c_char_p, c.c_char_p, c.c_int64]
-    return lib
-
-
-def ref_biaser(ref, blob, terms):
-    tok = ref.ref_tokenizer_new_bpe(blob, len(blob))
-    b = ref.ref_biaser_new()
-    for term in terms:
-        buf = ctypes.create_string_buffer(1024)
-        n = ref.ref_biaser_variants(term.encode(), buf, 1024)
-        for variant in buf.raw.split(b"\0")[:n]:
-            ids = np.zeros(64, np.int32)
-            k = ref.ref_text_to_tokens(tok, variant, ids.ctypes.data_as(ctypes.POINTER(ctypes.c_int32)), 64)
-            assert k > 0
-            ref.ref_biaser_add(b, ids.ctypes.data_as(ctypes.POINTER(ctypes.c_int32)), k)
-    return b
-
-
-def biased_greedy(ref, o, d, memory, budget, biaser):
-    cross = o.cross_kv(memory)
-    cache = o.new_self_cache()
-    toks, cur = [d.bos], d.bos
-    ref.ref_biaser_reset(biaser)
-    for t in range(budget):
-        lg = np.ascontiguousarray(o.decoder_step([cur], t, cache, cross)[0], np.float32)
-        ref.ref_biaser_apply(biaser, lg.ctypes.data_as(ctypes.POINTER(ctypes.c_float)), d.vocab)
-        nxt = int(np.argmax(lg))
-        toks.append(nxt)
-        if nxt == d.eos:
-            break
-        ref.ref_biaser_advance(biaser, nxt)
-        cur = nxt
-    return toks
+    return reference_golden("ref_keyterms.json")
 
 
 def test_keyterm_bias_changes_the_transcript_like_the_reference_biaser(ref):
+    """`plain`: the oracle's unbiased greedy ids; `terms`: spelled from vocabulary pieces that decode does not produce,
+    each starting with the word-boundary marker so it has exactly one spelling (ContextBiaser::variants_for_term);
+    `biased`: the oracle's greedy ids with the reference biaser at its fixed default boost of 2."""
     arch = "test_streaming"
     d = ARCHS[arch]
-    blob = synth_tokenizer_bin(d.vocab)
-    vocab = orc.load_tokenizer_bin(blob)
-    audio = synth_audio(21, 16000 * 3)
-    seg = audio[: len(audio) // 512 * 512]
-    o = StreamingOracle(SDims.from_product(d), synth_weights(arch, 0))
-    n_feat = len(seg) // 1280 * 4
-    mem = o.memory_stateless(seg, n_feat, n_feat)
-    budget = o.max_tokens_greedy(len(seg))
-    plain, _ = o.greedy_memory(mem, budget, keep_logits=False)
-    # key terms spelled from vocabulary pieces the unbiased decode does not produce; each starts with the
-    # word-boundary marker, so it has exactly one spelling (ContextBiaser::variants_for_term)
-    marker = "▁".encode()
-    starts = [i for i in range(10, d.vocab - 3) if vocab[i].startswith(marker)
-              and all(j not in plain for j in (i, i + 1, i + 2))]
-    a, b = starts[0], starts[5]
-    terms = [(vocab[a] + vocab[a + 1]).decode(), (vocab[b] + vocab[b + 1] + vocab[b + 2]).decode()]
+    vocab = orc.load_tokenizer_bin(synth_tokenizer_bin(d.vocab))
+    audio = synth_audio(*KEYTERM_AUDIO)
+    plain, terms, want_default = ref["plain"], ref["terms"], ref["biased"]
     boost = 60.0
-    biaser = ref_biaser(ref, blob, terms)
-    # the reference biaser has a fixed default boost of 2; emulate the option by scaling through its API is not
-    # exposed in the shim, so compare at the default boost first, then at a large boost through the product only
-    want_default = biased_greedy(ref, o, d, mem, budget, biaser)
     t = api.Transcriber(model_arch=api.ModelArch.TEST_STREAMING,
                         options={"vad_threshold": "0", "keyterms": ",".join(terms)},
                         memory_files=memory_files(arch, 0))
@@ -104,7 +40,8 @@ def test_keyterm_bias_changes_the_transcript_like_the_reference_biaser(ref):
     t.set_keyterms([])
     assert t.transcribe_without_streaming(audio).lines[0].text == orc.sanitize_utf8(orc.tokens_to_text(vocab, plain)).decode()
     t.close()
-    # a large boost forces the key terms into the transcript
+    # a large boost forces the key terms into the transcript (the reference biaser's boost is fixed, so this half is
+    # checked on the product alone)
     t2 = api.Transcriber(model_arch=api.ModelArch.TEST_STREAMING,
                          options={"vad_threshold": "0", "keyterms": ",".join(terms), "keyterm_boost": str(boost)},
                          memory_files=memory_files(arch, 0))

@@ -3,54 +3,26 @@ VoiceActivityDetector compiled from core/voice-activity-detector.cpp (oracle/_re
 replaced on both sides by a constant speech probability of 1.0.  Covers the documented bypass
 (`vad_threshold=0`), the smoothing window + max-segment fade at positive thresholds, look-behind across cuts,
 resampling, and audio fed in uneven pieces."""
-import ctypes
-import math
-import os
-
 import numpy as np
 import pytest
 
 from moonshine_b200 import api
-from oracle import build_ref
+from tests.util import digest, reference_golden
 
 
 @pytest.fixture(scope="module")
 def ref():
-    path = build_ref.build()
-    if path is None or not os.path.exists(path):
-        pytest.skip("oracle/_ref not built and /root/reference absent")
-    lib = ctypes.CDLL(path)
-    c = ctypes
-    lib.ref_vad_new.restype = c.c_void_p
-    lib.ref_vad_new.argtypes = [c.c_float, c.c_int32, c.c_int32, c.c_uint64, c.c_uint64]
-    for f in (lib.ref_vad_free, lib.ref_vad_start, lib.ref_vad_stop):
-        f.argtypes = [c.c_void_p]
-    lib.ref_vad_process.argtypes = [c.c_void_p, c.POINTER(c.c_float), c.c_uint64, c.c_int32]
-    lib.ref_vad_segment_count.restype = c.c_int32
-    lib.ref_vad_segment_count.argtypes = [c.c_void_p]
-    lib.ref_vad_segment.restype = c.c_int64
-    lib.ref_vad_segment.argtypes = [c.c_void_p, c.c_int32, c.POINTER(c.c_float), c.POINTER(c.c_float), c.c_int64]
-    return lib
+    return reference_golden("ref_segmentation.json")
 
 
-def ref_segments(ref, v):
-    out = []
-    for i in range(ref.ref_vad_segment_count(v)):
-        info = np.zeros(4, np.float32)
-        n = ref.ref_vad_segment(v, i, info.ctypes.data_as(ctypes.POINTER(ctypes.c_float)), None, 0)
-        audio = np.zeros(max(n, 1), np.float32)
-        ref.ref_vad_segment(v, i, info.ctypes.data_as(ctypes.POINTER(ctypes.c_float)),
-                            audio.ctypes.data_as(ctypes.POINTER(ctypes.c_float)), n)
-        out.append((float(info[0]), float(info[1]), bool(info[2]), audio[:n].copy()))
-    return out
-
-
-def make_ref_vad(ref, opts):
-    hop = int(opts.get("vad_hop_size", 512))
-    window = math.ceil(float(opts.get("vad_window_duration", 0.5)) * 16000 / hop)       # transcriber.cpp
-    max_seg = int(round(float(opts.get("vad_max_segment_duration", 15.0)) * 16000))
-    return ref.ref_vad_new(float(opts.get("vad_threshold", 0.5)), window, hop,
-                           int(opts.get("vad_look_behind_sample_count", 8192)), max_seg)
+def check_lines(lines, want):
+    """`want`: the reference detector's segments, [start_time, end_time, is_complete, sample count, SHA-256 of the
+    float32 samples] each."""
+    assert len(lines) == len(want)
+    for line, (st, en, complete, n, audio_sha) in zip(lines, want):
+        assert bool(line.is_complete) == complete
+        assert abs(line.start_time - st) < 1e-6 and abs(line.start_time + line.duration - en) < 1e-5
+        assert line.audio_data.size == n and digest(np.ascontiguousarray(line.audio_data, np.float32)) == audio_sha
 
 
 CASES = [
@@ -63,90 +35,79 @@ CASES = [
     ({"vad_threshold": "0"}, 44100 * 9 + 13, 44100),                      # resampled inside the VAD
     ({"vad_threshold": "0.5"}, 8000 * 30, 8000),
 ]
+CASE_IDS = [f"case{i}" for i in range(len(CASES))]
 
 
-@pytest.mark.parametrize("opts,n,rate", CASES, ids=[f"case{i}" for i in range(len(CASES))])
-def test_one_shot_segmentation_matches_reference_vad(ref, opts, n, rate):
+def one_shot_audio(n):
     rng = np.random.default_rng(n)
-    audio = (rng.standard_normal(n) * 0.05).astype(np.float32)
-    v = make_ref_vad(ref, opts)
-    ref.ref_vad_start(v)
-    ref.ref_vad_process(v, audio.ctypes.data_as(ctypes.POINTER(ctypes.c_float)), n, rate)
-    ref.ref_vad_stop(v)
-    want = ref_segments(ref, v)
-    ref.ref_vad_free(v)
+    return (rng.standard_normal(n) * 0.05).astype(np.float32)
+
+
+@pytest.mark.parametrize("opts,n,rate,case", [c + (i,) for c, i in zip(CASES, CASE_IDS)], ids=CASE_IDS)
+def test_one_shot_segmentation_matches_reference_vad(ref, opts, n, rate, case):
+    audio = one_shot_audio(n)
+    want = ref["one_shot"][case]
+    assert len(want) >= 1 and all(complete for _, _, complete, _, _ in want)
     o = {"skip_transcription": "true"}
     o.update(opts)
     t = api.Transcriber(None, api.ModelArch.TINY, o)
     tr = t.transcribe_without_streaming(audio, sample_rate=rate)
-    assert len(tr.lines) == len(want) and len(want) >= 1
-    for line, (st, en, complete, seg) in zip(tr.lines, want):
-        assert line.is_complete and complete
-        assert abs(line.start_time - st) < 1e-6 and abs(line.start_time + line.duration - en) < 1e-5
-        np.testing.assert_array_equal(line.audio_data, seg)
+    check_lines(tr.lines, want)
     t.close()
 
 
-@pytest.mark.parametrize("opts", [{"vad_threshold": "0"}, {}, {"vad_threshold": "0.7", "vad_max_segment_duration": "5"}],
-                         ids=["bypass", "default", "short_segments"])
-def test_streamed_segmentation_matches_reference_vad(ref, opts):
-    """Same audio fed in uneven pieces (hops straddle calls): after every update the lines equal the reference
-    detector's segments, including the still-open one."""
+STREAM_OPTS = {"bypass": {"vad_threshold": "0"}, "default": {},
+               "short_segments": {"vad_threshold": "0.7", "vad_max_segment_duration": "5"}}
+
+
+def streamed_pieces():
     rng = np.random.default_rng(5)
     audio = (rng.standard_normal(16000 * 26) * 0.05).astype(np.float32)
     cuts = np.sort(rng.choice(np.arange(1, len(audio)), 17, replace=False))
-    pieces = np.split(audio, cuts)
-    v = make_ref_vad(ref, opts)
-    ref.ref_vad_start(v)
+    return [np.ascontiguousarray(p) for p in np.split(audio, cuts)]
+
+
+@pytest.mark.parametrize("name", ["bypass", "default", "short_segments"])
+def test_streamed_segmentation_matches_reference_vad(ref, name):
+    """Same audio fed in uneven pieces (hops straddle calls): after every update the lines equal the reference
+    detector's segments, including the still-open one."""
+    pieces = streamed_pieces()
+    want = ref["streamed"][name]
+    assert len(want) == len(pieces)
     o = {"skip_transcription": "true"}
-    o.update(opts)
+    o.update(STREAM_OPTS[name])
     t = api.Transcriber(None, api.ModelArch.TINY, o)
     s = t.create_stream()
     s.start()
-    for p in pieces:
-        p = np.ascontiguousarray(p)
-        ref.ref_vad_process(v, p.ctypes.data_as(ctypes.POINTER(ctypes.c_float)), len(p), 16000)
+    for p, w in zip(pieces, want):
         s.add_audio(p)
-        tr = s.update_transcription(api.MOONSHINE_FLAG_FORCE_UPDATE)
-        want = ref_segments(ref, v)
-        assert len(tr.lines) == len(want)
-        for line, (st, en, complete, seg) in zip(tr.lines, want):
-            assert bool(line.is_complete) == complete
-            assert abs(line.start_time - st) < 1e-6 and abs(line.start_time + line.duration - en) < 1e-5
-            np.testing.assert_array_equal(line.audio_data, seg)
+        check_lines(s.update_transcription(api.MOONSHINE_FLAG_FORCE_UPDATE).lines, w)
     s.close()
     t.close()
-    ref.ref_vad_free(v)
 
 
-@pytest.mark.parametrize("opts", [{}, {"vad_threshold": "0.7", "vad_max_segment_duration": "5"}, {"vad_threshold": "0"}],
-                         ids=["default", "short_segments", "bypass"])
-def test_restarted_stream_matches_reference_vad(ref, opts):
-    """stop() + start() on the same stream: the reference's start() leaves the probability smoothing window as
-    it was (resize on an already-sized vector), so the second session's first segments open earlier than on a
-    fresh stream.  Compared segment by segment after the restart."""
+def restart_sessions():
     rng = np.random.default_rng(11)
     first = (rng.standard_normal(16000 * 7 + 123) * 0.05).astype(np.float32)
     second = (rng.standard_normal(16000 * 12 + 7) * 0.05).astype(np.float32)
-    v = make_ref_vad(ref, opts)
+    return first, second
+
+
+@pytest.mark.parametrize("name", ["default", "short_segments", "bypass"])
+def test_restarted_stream_matches_reference_vad(ref, name):
+    """stop() + start() on the same stream: the reference's start() leaves the probability smoothing window as
+    it was (resize on an already-sized vector), so the second session's first segments open earlier than on a
+    fresh stream.  Compared segment by segment after the restart."""
+    want = ref["restarted"][name]
     o = {"skip_transcription": "true"}
-    o.update(opts)
+    o.update(STREAM_OPTS[name])
     t = api.Transcriber(None, api.ModelArch.TINY, o)
     s = t.create_stream()
-    for audio in (first, second):
-        ref.ref_vad_start(v)
+    for audio, w in zip(restart_sessions(), want):
         s.start()
-        ref.ref_vad_process(v, audio.ctypes.data_as(ctypes.POINTER(ctypes.c_float)), len(audio), 16000)
         s.add_audio(audio)
-        tr = s.update_transcription(api.MOONSHINE_FLAG_FORCE_UPDATE)
-        want = ref_segments(ref, v)
-        assert len(tr.lines) == len(want) and len(want) >= 1
-        for line, (st, en, complete, seg) in zip(tr.lines, want):
-            assert bool(line.is_complete) == complete
-            assert abs(line.start_time - st) < 1e-6 and abs(line.start_time + line.duration - en) < 1e-5
-            np.testing.assert_array_equal(line.audio_data, seg)
-        ref.ref_vad_stop(v)
+        assert len(w) >= 1
+        check_lines(s.update_transcription(api.MOONSHINE_FLAG_FORCE_UPDATE).lines, w)
         s.stop()
     s.close()
     t.close()
-    ref.ref_vad_free(v)

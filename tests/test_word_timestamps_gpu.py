@@ -1,67 +1,24 @@
 """GPU: word timestamps through the reference ABI (`word_timestamps=true` -> transcript_line_t.words).
-Expected values: the oracle's decoder cross-attention fed to the REFERENCE's own align_words
-(oracle/_ref, compiled from core/word-alignment.cpp).  The GPU attention differs from the oracle's by ~1e-5,
-which can move a DTW boundary by a frame on a near-tie, so times are compared within two frames and
-required to be identical for most words."""
-import ctypes
-import os
-
+Expected values: the oracle's decoder cross-attention fed to the REFERENCE's own align_words (core/word-alignment.cpp),
+stored in golden/ref_word_timestamps.json by golden/make_golden_reference.py.  The GPU attention differs from the
+oracle's by ~1e-5, which can move a DTW boundary by a frame on a near-tie, so times are compared within two frames
+and required to be identical for most words."""
 import numpy as np
 import pytest
 
 from moonshine_b200 import api
-from moonshine_b200.arch import ARCHS
-from moonshine_b200.weights import synth_audio, synth_tokenizer_bin
-from oracle import build_ref
-from tests.util import memory_files, oracle_for
+from moonshine_b200.weights import synth_audio
+from tests.util import memory_files, reference_golden
 
 pytestmark = pytest.mark.gpu
+
+CLASSIC_CASES = [("test", 0, 48333), ("base", 0, 40000), ("tiny", 0, 80000)]
+STREAMING_AUDIO = (9, 16000 * 3 + 100)
 
 
 @pytest.fixture(scope="module")
 def ref():
-    path = build_ref.build()
-    if path is None or not os.path.exists(path):
-        pytest.skip("oracle/_ref not available")
-    lib = ctypes.CDLL(path)
-    c = ctypes
-    lib.ref_tokenizer_new.restype = c.c_void_p
-    lib.ref_tokenizer_new.argtypes = [c.c_char_p, c.c_uint64]
-    lib.ref_align_words.restype = c.c_int32
-    lib.ref_align_words.argtypes = [c.c_void_p, c.POINTER(c.c_float), c.c_int32, c.c_int32, c.c_int32, c.c_int32,
-                                    c.POINTER(c.c_int32), c.c_int32, c.c_float, c.POINTER(c.c_float),
-                                    c.POINTER(c.c_float), c.c_char_p, c.c_int64, c.c_int32]
-    return lib
-
-
-def oracle_words(ref, o, d, memory, tokens_budget, seg_samples, strip_eos=False):
-    """Greedy decode on `memory` collecting cross-attention, then the reference's align_words."""
-    cross = o.cross_kv(memory)
-    cache = o.new_self_cache()
-    toks, cur, att = [d.bos], d.bos, []
-    for t in range(tokens_budget):
-        lg, xa = o.decoder_step([cur], t, cache, cross, want_cross_attn=True)
-        att.append(np.stack([a[:, 0, :] for a in xa]))          # [L, H, T]
-        nxt = int(np.argmax(lg[0]))
-        toks.append(nxt)
-        if nxt == d.eos:
-            break
-        cur = nxt
-    steps, T = len(att), memory.shape[0]
-    x = np.stack(att, 2).reshape(d.dec_layers * d.heads, steps, T).astype(np.float32)   # [L*H, steps, T]
-    x = np.ascontiguousarray(x)
-    blob = synth_tokenizer_bin(d.vocab)
-    h = ref.ref_tokenizer_new(blob, len(blob))
-    ids = np.asarray(toks, np.int32)
-    st, en = np.zeros(256, np.float32), np.zeros(256, np.float32)
-    txt = ctypes.create_string_buffer(1 << 16)
-    tpf = np.float32(np.float32(seg_samples) / np.float32(16000.0)) / np.float32(T)
-    n = ref.ref_align_words(h, x.ctypes.data_as(ctypes.POINTER(ctypes.c_float)), d.dec_layers, d.heads, steps, T,
-                            ids.ctypes.data_as(ctypes.POINTER(ctypes.c_int32)), len(ids), tpf,
-                            st.ctypes.data_as(ctypes.POINTER(ctypes.c_float)),
-                            en.ctypes.data_as(ctypes.POINTER(ctypes.c_float)), txt, 1 << 16, 256)
-    words = [w.decode("utf-8") for w in txt.raw.split(b"\0")[:n]]
-    return words, st[:n].copy(), en[:n].copy(), float(tpf), toks
+    return reference_golden("ref_word_timestamps.json")
 
 
 def compare(line, words, st, en, tpf):
@@ -74,9 +31,8 @@ def compare(line, words, st, en, tpf):
     assert same.mean() >= 0.8, same.mean()
 
 
-@pytest.mark.parametrize("arch,seed,n", [("test", 0, 48333), ("base", 0, 40000), ("tiny", 0, 80000)])
+@pytest.mark.parametrize("arch,seed,n", CLASSIC_CASES)
 def test_word_timestamps_classic(ref, arch, seed, n):
-    d = ARCHS[arch]
     audio = synth_audio(7, n)
     t = api.Transcriber(model_arch={"test": api.ModelArch.TEST, "base": api.ModelArch.BASE,
                                     "tiny": api.ModelArch.TINY}[arch],
@@ -84,28 +40,19 @@ def test_word_timestamps_classic(ref, arch, seed, n):
                         memory_files=memory_files(arch, seed))
     tr = t.transcribe_without_streaming(audio)
     assert len(tr.lines) == 1
-    seg = audio[: len(audio) // 512 * 512]
-    o = oracle_for(arch, seed)
-    words, st, en, tpf, toks = oracle_words(ref, o, d, o.encoder(seg), o.max_len(len(seg)), len(seg))
-    assert len(words) > 0
-    compare(tr.lines[0], words, st, en, tpf)
+    w = ref["classic"][f"{arch}_s{seed}_{n}"]
+    assert len(w["words"]) > 0
+    compare(tr.lines[0], w["words"], np.array(w["start"], np.float32), np.array(w["end"], np.float32), w["time_per_frame"])
     t.close()
 
 
 def test_word_timestamps_streaming_arch(ref):
-    from oracle.moonshine_streaming_oracle import SDims, StreamingOracle
-    from moonshine_b200.weights import synth_weights
     arch = "test_streaming"
-    d = ARCHS[arch]
-    audio = synth_audio(9, 16000 * 3 + 100)
+    audio = synth_audio(*STREAMING_AUDIO)
     t = api.Transcriber(model_arch=api.ModelArch.TEST_STREAMING,
                         options={"vad_threshold": "0", "word_timestamps": "true"}, memory_files=memory_files(arch, 0))
     tr = t.transcribe_without_streaming(audio)
-    seg = audio[: len(audio) // 512 * 512]
-    o = StreamingOracle(SDims.from_product(d), synth_weights(arch, 0))
-    n_feat = len(seg) // 1280 * 4
-    mem = o.memory_stateless(seg, n_feat, n_feat)
-    words, st, en, tpf, _ = oracle_words(ref, o, d, mem, o.max_tokens_greedy(len(seg)), len(seg))
-    assert len(words) > 0
-    compare(tr.lines[0], words, st, en, tpf)
+    w = ref["streaming"]
+    assert len(w["words"]) > 0
+    compare(tr.lines[0], w["words"], np.array(w["start"], np.float32), np.array(w["end"], np.float32), w["time_per_frame"])
     t.close()

@@ -1,4 +1,6 @@
 """Shared helpers for the parity tests."""
+import hashlib
+import json
 import os
 import tempfile
 
@@ -33,6 +35,18 @@ def memory_files(arch, seed=0, init="scaled", tokenizer=None):
 
 def beckett():
     return np.load(os.path.join(GOLD, "beckett_pcm16.npy")).astype(np.float32) / np.float32(32768.0)
+
+
+def reference_golden(name):
+    """Outputs of the original project's own code recorded by golden/make_golden_reference.py."""
+    with open(os.path.join(GOLD, name), encoding="utf-8") as f:
+        return json.load(f)
+
+
+def digest(data):
+    """SHA-256 of the exact bytes (of a numpy array's buffer, or of a bytes object): how bit-exact outputs too large
+    to store are kept in the golden files."""
+    return hashlib.sha256(data.tobytes() if isinstance(data, np.ndarray) else bytes(data)).hexdigest()
 
 
 def rel_err(a, b):
