@@ -274,7 +274,6 @@ struct Ctx {
   const float* rope;         // smem: cos[0..64) | sin[64..128) of this step's position
   float* bias;               // smem: staged FC1 bias chunk (2 * IC floats)
   unsigned char* xp;         // smem: bf16 hi/lo planes of a GEMV's activation tile (16 rows, K-major SW64)
-  int mma;                   // layer GEMVs on tcgen05 (plane-packed weights)
   float* xg;                 // smem: bf16 hi/lo planes of the logits x tile (aliases hs..red)
   int nx;                    // utterances per logits pass (multiple of 16, <= 64)
   uint32_t tmem;             // TMEM base (128 columns)
@@ -559,14 +558,14 @@ __device__ __forceinline__ void gemm_ring_mma(Ring& ring, Ctx& c, const float* x
 // Which GEMVs take the tensor-core path: measured on B200, the single issuing thread plus the plane conversion
 // cost ~2 us per call, which only pays off once the SIMT mapping is compute-heavy (tiles of >= 8 utterances)
 // and the block has K >= 64 (QKV, cross-Q, FC1, FC2; not the K = head_dim output projections).  Producers and consumers apply the same rule.
-__device__ __forceinline__ bool gemv_on_tensor_cores(int mma_enabled, int NB, int K) {
-  return mma_enabled && NB >= 8 && K >= 64;
+__device__ __forceinline__ bool gemv_on_tensor_cores(int NB, int K) {
+  return NB >= 8 && K >= 64;
 }
 
 template <int NB>
 __device__ __forceinline__ void gemm_ring(Ring& ring, Ctx& c, const float* x, int ldx, int K, int N,
                                           const float* __restrict__ bias, float* out, int ldo) {
-  if (gemv_on_tensor_cores(c.mma, NB, K)) {
+  if (gemv_on_tensor_cores(NB, K)) {
     gemm_ring_mma<NB>(ring, c, x, ldx, K, N, bias, out, ldo);
     return;
   }
@@ -758,7 +757,7 @@ __device__ __forceinline__ void produce_self(const DecoderParams& p, int l, int 
   const int h = item % H, b0 = (item / H) * NB;
   if (!tile_active(p, active, NB, b0)) return;
   const DecLayerWeights& w = p.layers[l];
-  if (gemv_on_tensor_cores(p.mma_gemv, NB, D)) produce_block_planes(ring, w.wqkvP + (size_t)h * plane_block_bytes(3 * hd, D), 3 * hd, D);
+  if (gemv_on_tensor_cores(NB, D)) produce_block_planes(ring, w.wqkvP + (size_t)h * plane_block_bytes(3 * hd, D), 3 * hd, D);
   else produce_block_f32(ring, w.wqkv + (int64_t)h * D * 3 * hd, D, 3 * hd);
   if (p.step > 0) {
     for (int b = 0; b < NB; b++) {
@@ -768,7 +767,7 @@ __device__ __forceinline__ void produce_self(const DecoderParams& p, int l, int 
       produce_block_f32(ring, p.vs + bh * p.Smax * hd, p.step, hd);   // V rows [0, step)
     }
   }
-  if (gemv_on_tensor_cores(p.mma_gemv, NB, hd)) produce_block_planes(ring, w.woP + (size_t)h * plane_block_bytes(D, hd), D, hd);
+  if (gemv_on_tensor_cores(NB, hd)) produce_block_planes(ring, w.woP + (size_t)h * plane_block_bytes(D, hd), D, hd);
   else produce_block_f32(ring, w.wo + (int64_t)h * hd * D, hd, D);
 }
 
@@ -924,7 +923,7 @@ __device__ __forceinline__ void produce_cross(const DecoderParams& p, int l, int
   const int h = item % H, b0 = (item / H) * NB;
   if (!tile_active(p, active, NB, b0)) return;
   const DecLayerWeights& w = p.layers[l];
-  if (gemv_on_tensor_cores(p.mma_gemv, NB, D)) produce_block_planes(ring, w.wqcP + (size_t)h * plane_block_bytes(hd, D), hd, D);
+  if (gemv_on_tensor_cores(NB, D)) produce_block_planes(ring, w.wqcP + (size_t)h * plane_block_bytes(hd, D), hd, D);
   else produce_block_f32(ring, w.wqc + (int64_t)h * D * hd, D, hd);
   for (int b = 0; b < NB; b++) {
     if (b0 + b >= p.B || !active[b0 + b]) continue;
@@ -932,7 +931,7 @@ __device__ __forceinline__ void produce_cross(const DecoderParams& p, int l, int
     produce_block_f16(ring, p.kc + bh * hd * p.Tpad, hd, p.Tpad);   // K^T [hd][Tpad]
     produce_block_f16(ring, p.vc + bh * p.Tpad * hd, p.Tpad, hd);   // V   [Tpad][hd]
   }
-  if (gemv_on_tensor_cores(p.mma_gemv, NB, hd)) produce_block_planes(ring, w.wocP + (size_t)h * plane_block_bytes(D, hd), D, hd);
+  if (gemv_on_tensor_cores(NB, hd)) produce_block_planes(ring, w.wocP + (size_t)h * plane_block_bytes(D, hd), D, hd);
   else produce_block_f32(ring, w.woc + (int64_t)h * hd * D, hd, D);
 }
 
@@ -1097,9 +1096,9 @@ __device__ __forceinline__ void produce_mlp(const DecoderParams& p, int l, int i
   const int ch = item % p.n_chunk, b0 = (item / p.n_chunk) * NB;
   if (!tile_active(p, active, NB, b0)) return;
   const DecLayerWeights& w = p.layers[l];
-  if (gemv_on_tensor_cores(p.mma_gemv, NB, D)) produce_block_planes(ring, w.w1P + (size_t)ch * plane_block_bytes(2 * IC, D), 2 * IC, D);
+  if (gemv_on_tensor_cores(NB, D)) produce_block_planes(ring, w.w1P + (size_t)ch * plane_block_bytes(2 * IC, D), 2 * IC, D);
   else produce_block_f32(ring, w.w1 + (int64_t)ch * D * 2 * IC, D, 2 * IC);
-  if (gemv_on_tensor_cores(p.mma_gemv, NB, IC)) produce_block_planes(ring, w.w2P + (size_t)ch * plane_block_bytes(D, IC), D, IC);
+  if (gemv_on_tensor_cores(NB, IC)) produce_block_planes(ring, w.w2P + (size_t)ch * plane_block_bytes(D, IC), D, IC);
   else produce_block_f32(ring, w.w2 + (int64_t)ch * IC * D, IC, D);
 }
 
@@ -1416,7 +1415,6 @@ decoder_step2_kernel(const __grid_constant__ DecoderParams p) {
     c.nx = logits_rows_per_pass(p.B, p.D, L.xg_bytes);
     c.tmem = tmem_base;
     c.xp = smem_raw + L.xp;
-    c.mma = p.mma_gemv;
     c.acc_bar = bars + 32;
     c.acc_phase = 0;
   }

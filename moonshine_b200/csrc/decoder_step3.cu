@@ -344,7 +344,6 @@ struct Ctx {
   unsigned char* xp;         // smem: x planes of an attention job (16 rows)
   unsigned char* xg;         // smem: x planes of a GEMM job / logits pass (aliases the attention scratch)
   uint32_t tmem;             // TMEM base (256 columns)
-  int mma3;                  // experiment: 3 MMAs of N = NXp per k16 step instead of 2 (N = 2 NXp, NXp)
   uint64_t* acc_bar;         // accumulator-ready mbarrier
   int acc_phase;
   unsigned long long* prof;  // optional [grid][kProfSlots] stamps (thread 0)
@@ -544,6 +543,8 @@ __device__ __forceinline__ void gemm_block(Ring& ring, Ctx& c, const unsigned ch
         const uint32_t a_base = uniform_u32(smem_u32(ring.data + (size_t)ring.stage() * kStageBytes));
         const uint32_t empty_bar = uniform_u32(smem_u32(&ring.empty[ring.stage()]));
         if (elect_one()) {
+          // not unrolled: the kernel's code already overflows the instruction cache (DESIGN.md 4.2)
+#pragma unroll 1
           for (int q = 0; q < n; q++) {
             const int kb = kb0 + q;
             const uint32_t a_hi = a_base + (uint32_t)(q * Rp * 128), a_lo = a_hi + (uint32_t)(Rp * 64);
@@ -553,14 +554,8 @@ __device__ __forceinline__ void gemm_block(Ring& ring, Ctx& c, const unsigned ch
               if (kb * 32 + ks * 16 >= K) break;  // nothing but zero padding beyond K
               const uint32_t ko = (uint32_t)ks * 32u;
               const uint32_t acc = (kb | ks) ? 1u : 0u;
-              if (c.mma3) {  // experiment knob (MOONSHINE_B200_DECODER_GEMV=mma3): three N = NXp products
-                umma_bf16(tmem_d, make_desc_sw64(a_hi + ko), make_desc_sw64(b_hi + ko), idesc, acc);
-                umma_bf16(tmem_d + NXp, make_desc_sw64(a_hi + ko), make_desc_sw64(b_hi + (uint32_t)(NXp * 64) + ko), idesc, acc);
-                umma_bf16(tmem_d + 2 * NXp, make_desc_sw64(a_lo + ko), make_desc_sw64(b_hi + ko), idesc, acc);
-              } else {
-                umma_bf16(tmem_d, make_desc_sw64(a_hi + ko), make_desc_sw64(b_hi + ko), idesc2, acc);
-                umma_bf16(tmem_d + 2 * NXp, make_desc_sw64(a_lo + ko), make_desc_sw64(b_hi + ko), idesc, acc);
-              }
+              umma_bf16(tmem_d, make_desc_sw64(a_hi + ko), make_desc_sw64(b_hi + ko), idesc2, acc);
+              umma_bf16(tmem_d + 2 * NXp, make_desc_sw64(a_lo + ko), make_desc_sw64(b_hi + ko), idesc, acc);
             }
           }
           // warp 0's arrival on the stage: it is free once the MMAs have read it
@@ -980,8 +975,8 @@ __device__ __forceinline__ void produce_cross(const DecoderParams& p, int l, int
   // The cross K/V stream carries an L2 evict-first hint: the 191 MB a base/256 layer streams must not push the weight
   // planes out of L2 (measured 1677 -> 1582 us/step; an L2 prefetch window ahead of the ring and next-phase weight
   // prefetches were built and measured neutral or negative, profiles/r2e_prefetch_ab.txt, and removed again).
-  uint64_t pol = 0;
-  if (p.pf_mask & 32) asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
+  uint64_t pol;
+  asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
   produce_block_planes(ring, w.wqcP + (size_t)h * plane_block_bytes(hd, D), hd, D);
   for (int b = 0; b < nb; b++) {
     if (b0 + b >= p.B || !active[b0 + b]) continue;
@@ -1025,8 +1020,8 @@ __device__ void job_cross(const DecoderParams& p, int l, int job, Ctx& c, Ring& 
   // Tiles with an even number of utterances give the two halves of the CTA (4 warps each, own named barrier and scratch)
   // alternate utterances: while one half is in the softmax / PV of utterance b the other is already in the scores of
   // b + 1 -- the 112 threads that own 4 keys each are all a 448-key utterance can use in the scores pass anyway.
-  // Otherwise (one utterance per tile) the whole CTA walks it.  MOONSHINE_B200_CROSS_HALVES=0 restores pairs-only.
-  const bool halves = (nb >= 2) && ((nb & 1) == 0) && (Tpad <= 512) && (nb == 2 || p.cross_halves);
+  // Otherwise (one utterance per tile) the whole CTA walks it.
+  const bool halves = (nb >= 2) && ((nb & 1) == 0) && (Tpad <= 512);
   const int half = halves ? (int)(threadIdx.x >> 7) : 0;
   const int gtid = halves ? (int)(threadIdx.x & 127) : (int)threadIdx.x;
   const int gthreads = halves ? 128 : kConsumers;
@@ -1611,7 +1606,6 @@ __global__ void __launch_bounds__(kThreads3, 1) decoder_step3_kernel(const __gri
     c.rope = rope;
   }
   c.tmem = tmem_base;
-  c.mma3 = (int)uniform_u32((uint32_t)(p.mma_gemv == 2));
   c.acc_bar = bars + 32;
   c.acc_phase = 0;
   c.prof = reinterpret_cast<unsigned long long*>(p.prof);
@@ -1809,10 +1803,6 @@ bool decoder_step3_supported(const DecoderParams& p) {
 
 void decoder_step3_plan(DecoderParams& p, int grid) {
   const int B = p.B;
-  auto env_int = [](const char* name, int dflt) {
-    const char* e = std::getenv(name);
-    return e ? std::atoi(e) : dflt;
-  };
   // attention tiles: enough jobs to occupy ~128 CTAs, at most 16 utterances (one N = 16 operand)
   auto pick = [&](int want_jobs) {
     int nb = 1;
@@ -1826,19 +1816,13 @@ void decoder_step3_plan(DecoderParams& p, int grid) {
     if (p.row_group > kMaxNB || (kMaxNB % p.row_group) != 0) throw std::runtime_error("decoder v3: row group must divide 16");
     while (p.nb_self % p.row_group) p.nb_self *= 2;
   }
-  p.nb_self = env_int("MOONSHINE_B200_NB_SELF", p.nb_self);
-  p.nb_cross = env_int("MOONSHINE_B200_NB_CROSS", p.nb_cross);
-  auto pow2_le16 = [](int v) { return v == 1 || v == 2 || v == 4 || v == 8 || v == 16; };
-  if (!pow2_le16(p.nb_self) || !pow2_le16(p.nb_cross)) throw std::runtime_error("decoder v3: attention tiles must be 1, 2, 4, 8 or 16");
   // GEMM groups: 32 utterances (measured: 64 / 48 / 32 -> 1470 / 1471 / 1419 us per step at base/256, 767 -> 734 at
   // base-streaming/64: smaller groups mean more jobs per phase and shorter resolve prologues), fewer when the x planes of
   // the widest input would not fit 80 KB
   const int Kc = p.I / p.ffn_ksplit;
   const int kmax = (std::max(p.D, Kc) + 31) / 32 * 32;
-  int nx = std::min(32, (B + 15) & ~15);
-  while (nx > 16 && nx * kmax * 4 > 80 * 1024) nx -= 16;
-  p.nx = env_int("MOONSHINE_B200_NX", nx);
-  if (p.nx % 16 || p.nx < 16 || p.nx > 64) throw std::runtime_error("decoder v3: GEMM group must be 16, 32, 48 or 64");
+  p.nx = std::min(32, (B + 15) & ~15);
+  while (p.nx > 16 && p.nx * kmax * 4 > 80 * 1024) p.nx -= 16;
   // CTA assignment.  Small batches leave CTAs beyond the attention jobs: they become the GEMM engines (their
   // weight tiles sit in shared memory before the attention phases end).  Large batches spread every phase.
   const int ng = (B + p.nx - 1) / p.nx;

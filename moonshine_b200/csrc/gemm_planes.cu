@@ -647,10 +647,6 @@ void launch_gemm_planes(const GemmPlanesParams& p, cudaStream_t stream) {
   // Two mappings.  `tiles`: one 128 x 128 tile per CTA, 2 CTAs per SM -- best when a launch is only a few waves (tiny/32:
   // 105 row tiles).  `persistent`: 128 x 256 macro tiles, epilogue overlapped -- best from ~8 macro tiles per SM on
   // (base/256 encoder stage 27.2 -> 24.6 ms, base-streaming/64 7.0 -> 6.4; tiny/32 2.35 vs 2.49 the other way).
-  static const int forced = [] {
-    const char* e = std::getenv("MOONSHINE_B200_GEMM_PLANES");
-    return e == nullptr ? 0 : (std::string(e) == "tiles" ? 1 : (std::string(e) == "persistent" ? 2 : 0));
-  }();
   int dev = 0, sms = 148;
   cudaGetDevice(&dev);
   static int sm_count[64] = {0};
@@ -660,8 +656,7 @@ void launch_gemm_planes(const GemmPlanesParams& p, cudaStream_t stream) {
   }
   const int n_macro = ((p.N + 127) / 128 + 1) / 2, m_tiles = (p.M + 127) / 128;
   const int64_t total = (int64_t)n_macro * m_tiles;
-  const int want = p.variant ? p.variant : forced;
-  const bool tiles = want == 1 || (want == 0 && total < 8 * (int64_t)sms);
+  const bool tiles = p.variant == 1 || (p.variant == 0 && total < 8 * (int64_t)sms);
   if (tiles) {
     const size_t smem = 1024 + (size_t)kStages * kStage;
     static SmemAttrCache cache;

@@ -123,7 +123,7 @@ __device__ __forceinline__ void split4(const float4 v, uint2& hi, uint2& lo) {
   lo.y = *reinterpret_cast<const uint32_t*>(&l23);
 }
 
-__global__ void __launch_bounds__(kThreadsTC, 2) gemm_tc_kernel(const __grid_constant__ GemmParams p, const int dbg) {
+__global__ void __launch_bounds__(kThreadsTC, 2) gemm_tc_kernel(const __grid_constant__ GemmParams p) {
   const int z = blockIdx.z;
   const int Mz = p.Mz ? p.Mz[z] : p.M;
   const int Nz = p.Nz ? p.Nz[z] : p.N;
@@ -187,7 +187,7 @@ __global__ void __launch_bounds__(kThreadsTC, 2) gemm_tc_kernel(const __grid_con
       for (int i = 0; i < 8; i++) {
         const int rl = i * 16 + rsub;
         const int r = row0 + rl;
-        if (r < rows_valid && k < Kz && !(dbg & 2)) {
+        if (r < rows_valid && k < Kz) {
           const uint32_t d = smem_u32(dst + rl * 128 + q * 16);
           const float* g = src + (int64_t)r * ld + k;
           asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(d), "l"(g) : "memory");
@@ -208,7 +208,7 @@ __global__ void __launch_bounds__(kThreadsTC, 2) gemm_tc_kernel(const __grid_con
       for (int i = 0; i < 8; i++) {
         const int rl = i * 16 + rsub;
         const int r = row0 + rl;
-        if (r < rows_valid && k < Kz && !(dbg & 2)) {
+        if (r < rows_valid && k < Kz) {
           v[i] = *reinterpret_cast<const float4*>(rsrc + rl * 128 + q * 16);
           if (k + 3 >= Kz) {  // K tail inside the float4: row padding must not contribute
             if (k + 1 >= Kz) v[i].y = 0.f;
@@ -234,7 +234,7 @@ __global__ void __launch_bounds__(kThreadsTC, 2) gemm_tc_kernel(const __grid_con
         *reinterpret_cast<uint2*>(stage + off) = hi[i];
         *reinterpret_cast<uint2*>(stage + kTileBytes + off) = lo[i];
       }
-      if (!(dbg & 1)) asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic-proxy writes -> async proxy (UMMA)
+      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic-proxy writes -> async proxy (UMMA)
       mbar_arrive(&full_bar[s]);
     }
   } else {
@@ -272,7 +272,7 @@ __global__ void __launch_bounds__(kThreadsTC, 2) gemm_tc_kernel(const __grid_con
   // TMEM -> registers -> shared (row pitch 132 floats, conflict-free) -> coalesced row-wise
   // stores: 16 lanes cover 64 contiguous columns of one output row.  The staging area reuses
   // the operand ring, which is idle once the accumulator barrier has fired.
-  if (warp < 8 && !(dbg & 4)) {
+  if (warp < 8) {
     mbar_wait(&accum_bar, 0);
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     const int64_t c_base = p.offC ? p.offC[z] : (int64_t)z * p.strideC;
@@ -335,8 +335,7 @@ void launch_gemm_tc(const GemmParams& p, cudaStream_t stream) {
   if (cache.needs(smem))
     CUDA_CHECK(cudaFuncSetAttribute(gemm_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   dim3 grid((p.N + TN - 1) / TN, (p.M + TM - 1) / TM, p.groups);
-  static const int dbg = std::getenv("MOONSHINE_B200_GEMM_DBG") ? std::atoi(std::getenv("MOONSHINE_B200_GEMM_DBG")) : 0;
-  gemm_tc_kernel<<<grid, kThreadsTC, smem, stream>>>(p, dbg);
+  gemm_tc_kernel<<<grid, kThreadsTC, smem, stream>>>(p);
 }
 
 void launch_gemm(const GemmParams& p, cudaStream_t stream) {

@@ -234,11 +234,10 @@ struct DecoderParams {
   DecLayerWeights layers[kMaxDecLayers];
   const float* embed;     // [V][D]   (gather)
   const float* embT;      // [D][V]   (tied logits head, k-major)
-  const void* embP;       // v2 logits slab: bf16 hi/lo planes in UMMA K-major SWIZZLE_64B order,
+  const void* embP;       // v2-v4 logits slab: bf16 hi/lo planes in UMMA K-major SWIZZLE_64B order,
                           // [n_vchunk][m-tile][k-block of 32][plane][rows][32] (see Model::build_weights)
-  int smem_limit;         // opt-in shared memory per CTA (v2 ring sizing)
-  int mma_gemv;           // v2: layer GEMVs on tcgen05 from the plane-packed blocks (else fp32 SIMT from the k-major ones)
-  void* prof;             // optional [grid][512] u64 timestamps (v2 kernel, debugging)
+  int smem_limit;         // opt-in shared memory per CTA (v2-v4 shared-memory layouts)
+  void* prof;             // optional [grid][512] u64 timestamps (v2-v4 kernels, debugging)
   const float* final_ln;  // [D]
   const float* rope_cos;  // [Smax][rot/2]
   const float* rope_sin;
@@ -273,8 +272,6 @@ struct DecoderParams {
   // sparse logit bonuses added in the logits epilogue before the fused argmax (key-term biasing,
   // reference: ContextBiaser::apply, core/context-biaser.cpp:88-132); all null = no biasing
   int c4_cs, c4_nc, c4_u;     // v4: cluster size, clusters, utterances per cluster
-  int cross_halves;           // v3: the two halves of a CTA alternate the utterances of a cross-attention tile (default on)
-  int pf_mask;                // bit 5 (32): L2 evict-first hint on the v3 cross K/V stream (the L2 prefetch experiments of round 2 -- bits 0-4 -- measured neutral or negative and were removed, profiles/r2e_prefetch_ab.txt)
   // ---- explicit rows (v3 only; multi-token verify and per-utterance positions; reference: run_decoder_with_cross_kv
   // fed n > 1 tokens by decode_tokens / decode_full, core/moonshine-streaming-model.cpp:1136-1190, 1192-1397).  A row is
   // one (utterance, position) pair; rows of one utterance are consecutive, ascending in position, and never straddle a

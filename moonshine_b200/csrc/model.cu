@@ -9,7 +9,6 @@
 #include <cmath>
 #include <chrono>
 #include <cstring>
-#include <thread>
 
 namespace msb {
 
@@ -125,18 +124,11 @@ Model::Model(const Dims& dims, const WeightFile& weights, int device) : d_(dims)
   if (d_.dec_layers > kMaxDecLayers) throw std::runtime_error("too many decoder layers");
   CUDA_CHECK(cudaDeviceGetAttribute(&smem_optin_, cudaDevAttrMaxSharedMemoryPerBlockOptin, device_));
   {
-    const char* e = std::getenv("MOONSHINE_B200_DECODER");
-    decoder_v2_ = !(e && std::string(e) == "v1");
-    decoder_v3_ = !(e && (std::string(e) == "v1" || std::string(e) == "v2"));
-  }
-  {
     // v4 (cluster-resident layers) serves small batches of small models: every cluster streams all layer weights,
     // so they have to stay L2-resident next to the streamed cross K/V
-    const char* e = std::getenv("MOONSHINE_B200_DECODER");
-    const bool want_v4 = decoder_v3_ && !(e && std::string(e) == "v3");
     const double layer_mb = (double)d_.dec_layers * (4.0 * d_.dim * d_.dim + 3.0 * d_.dim * d_.ffn) * 4.0 / 1e6;
     c4_cs_ = 0;
-    if (want_v4 && layer_mb <= 48.0 && d_.dim % 32 == 0)
+    if (layer_mb <= 48.0 && d_.dim % 32 == 0)
       c4_cs_ = decoder_step4_cluster_size(device_, d_.heads, (size_t)smem_optin_, &c4_nc_);
     if (c4_cs_ > 0 && (d_.dim % c4_cs_ || d_.ffn % c4_cs_ || ((2 * d_.ffn / c4_cs_) % 4) || c4_cs_ % d_.heads)) c4_cs_ = 0;
   }
@@ -165,7 +157,6 @@ Model::Model(const Model& src, int device) : d_(src.d_), device_(device) {
   CUDA_CHECK(cudaStreamCreateWithFlags(&stream_, cudaStreamNonBlocking));
   for (auto& e : ev_) CUDA_CHECK(cudaEventCreate(&e));
   CUDA_CHECK(cudaDeviceGetAttribute(&smem_optin_, cudaDevAttrMaxSharedMemoryPerBlockOptin, device_));
-  decoder_v2_ = src.decoder_v2_; decoder_v3_ = src.decoder_v3_;
   ffn_chunk_ = src.ffn_chunk_; ffn_ksplit_ = src.ffn_ksplit_; vchunk_ = src.vchunk_; n_vchunk_ = src.n_vchunk_;
   s_k_ = src.s_k_;
   c4_cs_ = src.c4_cs_; c4_nc_ = src.c4_nc_;
@@ -347,7 +338,6 @@ void Model::build_weights(const WeightFile& wf) {
   {
     const int Ee = d_.streaming ? d_.enc_dim : D, EIe = d_.streaming ? d_.enc_ffn : I;
     enc_planes_ = Ee % 32 == 0 && EIe % 32 == 0 && Ee <= 512;
-    if (const char* e = std::getenv("MOONSHINE_B200_ENC")) enc_planes_ = enc_planes_ && std::string(e) != "classic";
     // (the decoder's stacked cross K | V projections [2 L D][D] are packed after the decoder weights are laid out)
     if (enc_planes_ && !d_.streaming) {  // conv2 [2D][7D] and conv3 [D][6D] (tap-major K, as the fp32 copies)
       const size_t c2 = o_c2, c3 = o_c3;
@@ -387,11 +377,11 @@ void Model::build_weights(const WeightFile& wf) {
   // planes, laid out exactly as the UMMA K-major SWIZZLE_64B shared-memory tiles the kernel issues
   // MMAs on: [vocab chunk][m-tile of <=128 rows][k-block of 32][plane hi|lo][row][32 bf16], the 16-byte
   // chunk c of row r stored at position c ^ ((r >> 1) & 3).  A ring stage receives it by one bulk copy.
-  if (D % 32 != 0 && decoder_v2_) decoder_v2_ = false;  // v2 needs whole 32-wide k-blocks
+  const bool dec_tc_layouts = D % 32 == 0;  // the tensor-core decoders (v2, v3, v4) need whole 32-wide k-blocks
   const int n_mt = (vchunk_ + 127) / 128;
   const size_t slab_halfs = (size_t)n_vchunk_ * vchunk_ * D * 2;  // hi + lo
   size_t o_embP = bb.add((slab_halfs + 1) / 2);
-  if (decoder_v2_) {
+  if (dec_tc_layouts) {
     uint16_t* P = reinterpret_cast<uint16_t*>(&bb.data[o_embP]);
     auto bf16_rn = [](float x) -> uint16_t {
       uint32_t u; std::memcpy(&u, &x, 4);
@@ -500,7 +490,7 @@ void Model::build_weights(const WeightFile& wf) {
         for (int n = 0; n < D; n++) w2[(size_t)kk * D + n] = f2[(size_t)n * I + c * IC + kk];
     }
     // tensor-core copies of the same blocks (v2 kernel); LayerNorm gammas folded in exactly as above
-    if (decoder_v2_) {
+    if (dec_tc_layouts) {
       // blocks of one kind are laid out back to back (block h at base + h * decoder_plane_bytes(N, K))
       for (int h = 0; h < H; h++) {
         const size_t a = pack_planes(bb, 3 * hd, D, [&](int n, int kk) {
@@ -534,7 +524,7 @@ void Model::build_weights(const WeightFile& wf) {
       }
     }
     // v3 kernel: whole matrices as 128-row m-tiles (weight-stationary GEMM jobs)
-    if (decoder_v2_) {
+    if (dec_tc_layouts) {
       dof[l].wocF = pack_planes(bb, D, D, [&](int n, int kk) { return oc[(size_t)n * D + kk]; });
       // fc1 rows interleaved (2j = value j, 2j+1 = gate j): the SiLU gate pairs adjacent TMEM lanes
       dof[l].w1iF = pack_planes(bb, 2 * I, D, [&](int n, int kk) {
@@ -626,19 +616,8 @@ void Model::build_weights(const WeightFile& wf) {
   dec_.D = D; dec_.H = H; dec_.hd = hd; dec_.I = I; dec_.V = V; dec_.L = d_.dec_layers;
   dec_.rot_dim = d_.rot_dim; dec_.IC = IC; dec_.n_chunk = n_chunk; dec_.ffn_ksplit = ffn_ksplit_;
   dec_.c4_cs = c4_cs_; dec_.c4_nc = c4_nc_;
-  {
-    const char* e = std::getenv("MOONSHINE_B200_PREFETCH");  // experiment knob (bit mask, see DecoderParams::pf_mask); default 32 = evict-first hint on v3's cross K/V stream (base/256 1677 -> 1582 us/step, base-streaming/64 842 -> 776); the prefetch bits measured neutral or negative (profiles/r2e_prefetch_ab.txt)
-    dec_.pf_mask = e ? std::atoi(e) : 32;
-    const char* ch = std::getenv("MOONSHINE_B200_CROSS_HALVES");
-    dec_.cross_halves = !(ch && ch[0] == '0');
-  }
   dec_.embed = base + o_emb; dec_.embT = base + o_embT; dec_.final_ln = base + o_decln;
   dec_.embP = base + o_embP; dec_.vchunk = vchunk_; dec_.n_vchunk = n_vchunk_; dec_.smem_limit = smem_optin_;
-  {
-    const char* e = std::getenv("MOONSHINE_B200_DECODER_GEMV");
-    dec_.mma_gemv = !(e && std::string(e) == "simt");
-    if (e && std::string(e) == "mma3") dec_.mma_gemv = 2;  // v3 experiment knob
-  }
   for (int l = 0; l < d_.dec_layers; l++) {
     DecLayerWeights& w = dec_.layers[l];
     w.ln1 = base + dof[l].ln1; w.wqkv = base + dof[l].wqkv; w.wo = base + dof[l].wo;
@@ -646,7 +625,7 @@ void Model::build_weights(const WeightFile& wf) {
     const unsigned char* bytes = reinterpret_cast<const unsigned char*>(base);
     w.wqkvP = bytes + dof[l].wqkvP * 4; w.woP = bytes + dof[l].woP * 4; w.wqcP = bytes + dof[l].wqcP * 4;
     w.wocP = bytes + dof[l].wocP * 4; w.w1P = bytes + dof[l].w1P * 4; w.w2P = bytes + dof[l].w2P * 4;
-    w.wocF = decoder_v2_ ? bytes + dof[l].wocF * 4 : nullptr; w.w1iF = bytes + dof[l].w1iF * 4;
+    w.wocF = dec_tc_layouts ? bytes + dof[l].wocF * 4 : nullptr; w.w1iF = bytes + dof[l].w1iF * 4;
     w.b1i = base + dof[l].b1i; w.w2kF = bytes + dof[l].w2kF * 4;
     if (c4_cs_ > 0) {
       w.c4_wo = base + dof[l].c4_wo; w.c4_woc = base + dof[l].c4_woc; w.c4_w1 = base + dof[l].c4_w1;
@@ -728,15 +707,6 @@ static void stream_copy(float* dst, const float* src, size_t n) {
 #endif
 }
 
-static bool nt_stores() {
-  static const bool on = [] { const char* e = std::getenv("MOONSHINE_B200_STAGE_NT"); return !(e && e[0] == '0'); }();
-  return on;
-}
-static int stage_mode() {  // experiment knob MOONSHINE_B200_STAGE: 0 threads + per-slice DMA, 1 pool + per-slice DMA, 2 pool + one DMA
-  static const int m = [] { const char* e = std::getenv("MOONSHINE_B200_STAGE"); return e ? std::atoi(e) : 2; }();
-  return m;
-}
-
 void Model::transcribe(const float* const* pcm, const uint64_t* n_samples, int B, float max_tps,
                        std::vector<std::vector<int32_t>>& tokens, DebugCapture* dbg, const StreamPlan* plan,
                        std::vector<CrossAttention>* xattn, LogitHook* hook) {
@@ -753,77 +723,22 @@ void Model::transcribe(const float* const* pcm, const uint64_t* n_samples, int B
   const auto t0 = std::chrono::steady_clock::now();
   for (int b = 0; b < B; b++)
     if (pcm[b] == nullptr && n_samples[b] > 0) throw std::runtime_error("Audio data is nullptr");
-  // Stage through pinned memory on the persistent worker pool (one memcpy thread moves ~5 GB/s, PCIe 5 x16 ~50) and start
-  // each slice's DMA as soon as it is staged: rows of a slice are contiguous in both buffers, the DMAs are issued in order
-  // by this thread as the slices complete.
+  // Stage through pinned memory, then ONE host-to-device DMA.  Large batches stage on the persistent worker pool (one
+  // memcpy thread moves ~5 GB/s, PCIe 5 x16 ~50); the DMA waits for all of it, since a copy engine reading lines other
+  // cores are still writing is slow.
   {
     const size_t total_bytes = (size_t)B * stride * sizeof(float);
     if (total_bytes < ((size_t)2 << 20) || B < 2) {
       for (int b = 0; b < B; b++) std::memcpy(pin_pcm_.ptr + (size_t)b * stride, pcm[b], n_samples[b] * sizeof(float));
-      CUDA_CHECK(cudaMemcpyAsync(pcm_dev_.ptr, pin_pcm_.ptr, total_bytes, cudaMemcpyHostToDevice, stream_));
-    } else if (stage_mode() == 2) {
-      // stage everything on the pool, then ONE DMA (a copy engine reading lines other cores are still writing is slow)
-      const int n_slices = std::min(B, 16);
-      const int per = (B + n_slices - 1) / n_slices;
-      WorkerPool::instance().parallel_for(n_slices, [&](int i) {
-        const int lo = i * per, hi = std::min(B, lo + per);
-        for (int b = lo; b < hi; b++) {
-          if (nt_stores()) stream_copy(pin_pcm_.ptr + (size_t)b * stride, pcm[b], (size_t)n_samples[b]);
-          else std::memcpy(pin_pcm_.ptr + (size_t)b * stride, pcm[b], n_samples[b] * sizeof(float));
-        }
-      });
-      CUDA_CHECK(cudaMemcpyAsync(pcm_dev_.ptr, pin_pcm_.ptr, total_bytes, cudaMemcpyHostToDevice, stream_));
-    } else if (stage_mode() == 0) {
-      const int nthreads = std::min(8, B);
-      auto stage_rows = [&](int lo, int hi) {
-        for (int b = lo; b < hi; b++)
-          std::memcpy(pin_pcm_.ptr + (size_t)b * stride, pcm[b], n_samples[b] * sizeof(float));
-      };
-      std::vector<std::thread> pool;
-      std::vector<std::pair<int, int>> slices;
-      const int per = (B + nthreads - 1) / nthreads;
-      for (int lo = 0; lo < B; lo += per) slices.emplace_back(lo, std::min(B, lo + per));
-      for (auto& sl : slices) pool.emplace_back(stage_rows, sl.first, sl.second);
-      for (size_t i = 0; i < slices.size(); i++) {
-        pool[i].join();
-        const size_t off = (size_t)slices[i].first * stride;
-        const size_t cnt = (size_t)(slices[i].second - slices[i].first) * stride;
-        CUDA_CHECK(cudaMemcpyAsync(pcm_dev_.ptr + off, pin_pcm_.ptr + off, cnt * sizeof(float),
-                                   cudaMemcpyHostToDevice, stream_));
-      }
     } else {
       const int n_slices = std::min(B, 16);
       const int per = (B + n_slices - 1) / n_slices;
-      std::vector<std::atomic<int>> ready(n_slices);
-      for (auto& r : ready) r.store(0);
-      std::exception_ptr dma_error;
-      std::atomic<int> issued{0};
-      std::mutex issue_mu;
-      // whoever finishes slice i tries to issue every DMA whose predecessors are all staged (in order, one issuer at a time)
-      auto issue_ready = [&]() {
-        std::lock_guard<std::mutex> lock(issue_mu);
-        while (issued.load() < n_slices && ready[issued.load()].load()) {
-          const int i = issued.load();
-          const int lo = i * per, hi = std::min(B, lo + per);
-          if (lo < hi && !dma_error) {
-            const size_t off = (size_t)lo * stride, cnt = (size_t)(hi - lo) * stride;
-            if (cudaMemcpyAsync(pcm_dev_.ptr + off, pin_pcm_.ptr + off, cnt * sizeof(float), cudaMemcpyHostToDevice, stream_) != cudaSuccess)
-              dma_error = std::make_exception_ptr(std::runtime_error("host-to-device copy of the staged audio failed"));
-          }
-          issued.fetch_add(1);
-        }
-      };
-      const int dev = device_;
       WorkerPool::instance().parallel_for(n_slices, [&](int i) {
         const int lo = i * per, hi = std::min(B, lo + per);
-        for (int b = lo; b < hi; b++)
-          std::memcpy(pin_pcm_.ptr + (size_t)b * stride, pcm[b], n_samples[b] * sizeof(float));
-        ready[i].store(1);
-        cudaSetDevice(dev);  // pool threads issue DMAs on this model's device
-        issue_ready();
+        for (int b = lo; b < hi; b++) stream_copy(pin_pcm_.ptr + (size_t)b * stride, pcm[b], (size_t)n_samples[b]);
       });
-      if (dma_error) std::rethrow_exception(dma_error);
     }
+    CUDA_CHECK(cudaMemcpyAsync(pcm_dev_.ptr, pin_pcm_.ptr, total_bytes, cudaMemcpyHostToDevice, stream_));
   }
   const auto t1 = std::chrono::steady_clock::now();
   run(pcm_dev_.ptr, stride, n_samples, B, max_tps, tokens, dbg, plan, xattn, hook);
@@ -1033,7 +948,7 @@ void Model::run(const float* d_pcm, int64_t stride, const uint64_t* n_samples, i
   reserve_zero(vt_, (size_t)B * E * Tp);
   {
     // only the unfused attention path materialises scores in HBM
-    bool need_scores = std::getenv("MOONSHINE_B200_ATTN") != nullptr;
+    bool need_scores = false;
     for (int l = 0; l < d_.enc_layers; l++)
       need_scores = need_scores || !attention_tc_supported(maxT3, ehd, S ? d_.win_past[l] : -1, S ? d_.win_future[l] : 0);
     if (need_scores) reserve_zero(scores_, (size_t)BH * maxT3 * Tp);
@@ -1127,10 +1042,6 @@ void Model::run(const float* d_pcm, int64_t stride, const uint64_t* n_samples, i
 
   // ---------------- encoder layers ----------------
   const float scale = 1.0f / std::sqrt((float)ehd);
-  static const bool fused_attn = [] {
-    const char* e = std::getenv("MOONSHINE_B200_ATTN");
-    return !(e && std::string(e) == "unfused");
-  }();
   for (int l = 0; l < d_.enc_layers; l++) {
     const EncLayer& w = enc_[l];
     unsigned char* lnP = reinterpret_cast<unsigned char*>(lnP_.ptr);
@@ -1167,7 +1078,7 @@ void Model::run(const float* d_pcm, int64_t stride, const uint64_t* n_samples, i
       launch_gemm(g, stream_);
     }
     const int wp = S ? d_.win_past[l] : -1, wf = S ? d_.win_future[l] : 0;
-    if (fused_attn && attention_tc_supported(maxT3, ehd, wp, wf)) {
+    if (attention_tc_supported(maxT3, ehd, wp, wf)) {
       // softmax(scale * Q K^T [window]) V in one tcgen05 kernel; scores stay in TMEM
       AttnParams a;
       a.qk = qk_.ptr; a.vt = vt_.ptr; a.out = attn_.ptr;
@@ -1371,11 +1282,12 @@ void Model::run(const float* d_pcm, int64_t stride, const uint64_t* n_samples, i
   const int grid = sm_count_;
   p.xattn_out = nullptr;
   p.xattn_steps = 0;
-  // v2 streams operands through the smem ring; its cross-attention maps one thread to 4 key
-  // positions, so clips longer than ~39 s (Tpad > 1024) take the v1 kernel.
-  const bool use_v2 = decoder_v2_ && Tpad <= 1024 && hd <= 64 && d_.rot_dim <= 128 && D % 32 == 0;
-  const bool use_v3 = use_v2 && decoder_v3_ && decoder_step3_supported(p);
+  // v2 streams operands through the smem ring; its cross-attention maps one thread to 4 key positions, so encoder
+  // memories longer than 1024 frames take the v1 kernel.  v3 and v4 share that limit and keep a LayerNorm row in
+  // registers, so they stop at D = 512: v2 serves the wider models.
+  const bool use_v3 = decoder_step3_supported(p);
   const bool use_v4 = use_v3 && c4_cs_ > 0 && decoder_step4_supported(p);
+  const bool use_v2 = !use_v3 && D % 32 == 0 && Tpad <= 1024 && hd <= 64 && d_.rot_dim <= 128;
   if (use_v4) decoder_step4_plan(p);
   else if (use_v3) decoder_step3_plan(p, grid);
   if (std::getenv("MOONSHINE_B200_VERBOSE"))
@@ -1394,16 +1306,14 @@ void Model::run(const float* d_pcm, int64_t stride, const uint64_t* n_samples, i
   }
   if (xattn != nullptr) {
     xattn->clear();
-    if (!use_v2)
-      throw std::runtime_error("word_timestamps: the cross-attention export needs the v2 decoder kernel "
-                               "(clips up to 39 s, head_dim <= 64, hidden size a multiple of 32)");
-    if (use_v2) {  // the export lives in the v2 step kernel
-      p.xattn_steps = std::max(max_steps, 1);
-      const size_t n = (size_t)B * L * H * p.xattn_steps * Tpad;
-      xattn_dev_.reserve(n);
-      CUDA_CHECK(cudaMemsetAsync(xattn_dev_.ptr, 0, n * sizeof(float), stream_));
-      p.xattn_out = xattn_dev_.ptr;
-    }
+    if (!use_v2 && !use_v3)
+      throw std::runtime_error("word_timestamps: the cross-attention export needs at most 1024 encoder frames, "
+                               "head_dim <= 64, rotary dimension <= 128 and a hidden size that is a multiple of 32");
+    p.xattn_steps = std::max(max_steps, 1);
+    const size_t n = (size_t)B * L * H * p.xattn_steps * Tpad;
+    xattn_dev_.reserve(n);
+    CUDA_CHECK(cudaMemsetAsync(xattn_dev_.ptr, 0, n * sizeof(float), stream_));
+    p.xattn_out = xattn_dev_.ptr;
   }
   std::vector<std::vector<int32_t>> hooked_tokens;  // filled by the host-stepped loop
   int steps_launched = max_steps;

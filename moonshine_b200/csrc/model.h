@@ -154,8 +154,6 @@ class Model {
   DecoderParams dec_{};  // weight pointers + dims prefilled
   int ffn_chunk_ = 64;
   int vchunk_ = 0, n_vchunk_ = 0, smem_optin_ = 0;
-  bool decoder_v2_ = true;
-  bool decoder_v3_ = true;
   int ffn_ksplit_ = 1;
   int c4_cs_ = 0;   // cluster size of the v4 decoder kernel (0: not used)
   int c4_nc_ = 0;   // co-resident clusters of that size

@@ -33,6 +33,18 @@ def test_no_cpu_fallback_in_the_model_path():
     assert not re.search(r"^\s*(import|from)\s+torch", api, re.M)  # the binding is ctypes over the C ABI, nothing else
 
 
+def test_environment_switches_are_the_kept_ones():
+    """The native code reads only these variables, each by its literal name: SPEC_VERIFY (the tests' A/B switch of draft
+    verification), V4_COOP (Nsight Compute cannot replay a launch that is both clustered and cooperative), PROF,
+    HOST_PROF, VERBOSE and DEBUG_SYNC (diagnostics that compute nothing differently) and GEMM=simt (every GEMM on the
+    exact fp32 SIMT reference).  A variable that selects between two paths does not belong in the product."""
+    names = set()
+    for path in _files(os.path.join("moonshine_b200", "csrc"), (".cpp", ".cu", ".h", ".cuh")):
+        names.update(a.strip() for a in re.findall(r"getenv\(([^)]*)\)", open(path, encoding="utf-8").read()))
+    kept = {"SPEC_VERIFY", "V4_COOP", "PROF", "HOST_PROF", "VERBOSE", "DEBUG_SYNC", "GEMM"}
+    assert names == {f'"MOONSHINE_B200_{k}"' for k in kept}, sorted(names)
+
+
 def test_header_symbols_are_all_exported():
     import ctypes
     from moonshine_b200 import api
